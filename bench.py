@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RoIs/s through the BAGS head fwd+bwd (1231 classes -> 1236 logits, 5 bins).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of 4096 synthetic RoIs per GPU
 (BASELINE.json configs[1]: 4096 RoIs x 1024 feat x 1231 cls, 5 bins, bf16):
@@ -22,6 +22,12 @@ One "step" = one pass of the hot path over one batch of 4096 synthetic RoIs per 
 
 --impl reference: the reference's own CPU implementation of the path (its source through
 oracle/ref_shim.py when a checkout is reachable, else the oracle port), same metric/config.
+
+--dump-outputs DIR: after the timed steps, what the last timed step returned to its caller -- the five per-bin
+losses, dW, db and dX of its buffer set -- as DIR/<name>.npy in float32 (see dump_outputs()).  Inputs, sampler
+seeds and the step schedule depend only on the arguments, so two builds run with the same arguments can be
+compared output for output.  The losses, db and dX repeat bit for bit from run to run; dW is summed split-K in
+fp32 in no fixed order, so its last bits vary (measured on a B200: ~5e-8 relative).
 """
 from __future__ import annotations
 
@@ -68,6 +74,28 @@ def ncu_traffic(kernel):
         return None if k is None else int(k['dram_read'] + k['dram_write'])
     except Exception:
         return None
+
+
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(directory, arrays, limit=DUMP_LIMIT_BYTES):
+    """Write each array as <directory>/<name>.npy in float32, at most `limit` bytes in all.  When the arrays are
+    larger than that together, every 2-D array keeps the same share of its rows: a sorted sample drawn with a fixed
+    seed, so that runs with the same arguments write the same rows."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    budget = limit - 1024 * len(arrays)           # room for the .npy headers
+    small = sum(a.nbytes for a in arrays.values() if a.ndim < 2)
+    large = sum(a.nbytes for a in arrays.values() if a.ndim >= 2)
+    share = 1.0 if large <= budget - small else (budget - small) / large
+    for name, a in arrays.items():
+        if a.ndim >= 2 and share < 1.0:
+            keep = max(1, int(a.shape[0] * share))
+            a = a[np.sort(np.random.RandomState(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(directory, name + '.npy'), a)
+    log('wrote %s to %s' % (', '.join(sorted(arrays)), directory))
 
 
 def make_labels(torch, n, num_classes, gen):
@@ -456,7 +484,7 @@ def run_ours(args):
                     do_exchange(side_stream)
                 do_dx()
             torch.cuda.current_stream(dev).wait_stream(side_stream)
-            last['loss'] = loss
+            last['loss'] = s['loss'] = loss
             return loss
         ops.fused_bwd(dz, s['x'], s['w'], gout, dt, colsum, dW=s['dW'], dX=s['dX'], wscratch=s['wscratch'],
                       db=s['db'], dw_prezeroed=prez)
@@ -477,7 +505,7 @@ def run_ours(args):
             ev.record(torch.cuda.current_stream(dev))
             comm_stream.wait_event(ev)
             nat.check(nat.lib().bags_debug_spin(fake[0], fake[1], fake[2], comm_stream.cuda_stream), 'bags_debug_spin')
-        last['loss'] = loss
+        last['loss'] = s['loss'] = loss
         return loss
 
     # sampler, fused fwd (or GEMM + grouped CE), merged backward (preparation jobs + dW + dX units in one launch)
@@ -547,6 +575,11 @@ def run_ours(args):
             dist.barrier()
         ms_total = e0.elapsed_time(e1)
         ms_step = ms_total / args.steps
+        if args.dump_outputs and rank == 0:
+            # step i of run_steps uses sets[i % pool]; nothing has touched the last one since
+            last_set = sets[(args.steps - 1) % pool]
+            dump_outputs(args.dump_outputs, {name: last_set[key].detach().float().cpu().numpy() for name, key in (
+                ('loss_bins', 'loss'), ('dW', 'dW'), ('db', 'db'), ('dX', 'dX'))})
         if world > 1:
             t = torch.tensor([ms_step], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -986,8 +1019,14 @@ def main():
     ap.add_argument('--unfused', action='store_true', help='GEMM -> fp32 logits -> grouped CE instead of the fused kernel')
     ap.add_argument('--no-library-baseline', action='store_true', help='skip the torch/cuBLAS same-GPU baseline leg')
     ap.add_argument('--profile', action='store_true', help='timed loop only (for ncu): skip e2e / cpu / per-kernel legs')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write the per-bin losses, dW, db and dX of the last timed step to DIR/<name>.npy (float32)')
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error('--steps must be at least 1')
     if args.impl == 'reference':
+        if args.dump_outputs:
+            ap.error('--dump-outputs applies to --impl ours')
         args.steps = args.steps or 20
         args.warmup = 3 if args.warmup is None else args.warmup
         return run_reference(args)

@@ -3,14 +3,15 @@
 The reference (FishYuLi/BalancedGroupSoftmax) cannot be installed here (needs
 mmcv, pycocotools and THC-era CUDA extensions), but the files on the hot path
 are plain PyTorch.  This shim loads them straight from a reference checkout
-(``$BAGS_REFERENCE_DIR``, ``/root/reference`` or ``baseline/_ref``) with
+(``$BAGS_REFERENCE_DIR`` or ``baseline/_ref``) with
 importlib, stubbing only what they import from outside the path (mmcv.is_str,
 mmdet.core.{bbox_target,delta2bbox,multiclass_nms}, ConvModule) and making
 ``Tensor.cuda()`` the identity so the head builds on CPU.  Nothing is copied
 into this repository.
 
-Used by tests (oracle validation) and by tests/golden/make_golden.py; never by
-the product.  ``available()`` is False on the GPU box (no checkout there).
+Used by tests/golden/make_golden.py (the reference outputs the tests compare
+against) and by the CPU arm of bench.py; never by the product.  ``available()``
+is False where no checkout is configured.
 """
 from __future__ import annotations
 
@@ -21,7 +22,7 @@ import tempfile
 import types
 from typing import Optional
 
-_CANDIDATES = [os.environ.get('BAGS_REFERENCE_DIR', ''), '/root/reference',
+_CANDIDATES = [os.environ.get('BAGS_REFERENCE_DIR', ''),
                os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'baseline', '_ref')]
 
 _loaded = None
